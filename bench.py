@@ -26,6 +26,7 @@ import math
 import os
 import subprocess
 import sys
+import tempfile
 import threading
 import time
 
@@ -355,8 +356,10 @@ def run_reference(args, rank, world):
         oracle.solve_batch(params, hb.slice(0, min(sample, 8 * threads)), nthreads=threads)
     t_tot = 0.0
     for _ in range(args.steps):
-        _, secs = oracle.solve_batch(params, hb, nthreads=threads, mode=0, dense_assembly=False)
+        res, secs = oracle.solve_batch(params, hb, nthreads=threads, mode=0, dense_assembly=False)
         t_tot += secs
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"sol": res.sol, "cost": res.cost, "status": res.status, "iters": res.iters})
     value = sample * args.steps / t_tot
     line = {
         "impl": "reference", "metric": METRIC, "value": value, "unit": UNIT, "n_gpus": args.gpus,
@@ -471,17 +474,34 @@ def bind_to_gpu_numa_node(local_rank):
         return None
 
 
+DUMP_BYTES = 64_000_000  # what --dump-outputs may write in all
+
+
+def dump_outputs(out_dir, arrays):
+    """--dump-outputs: the per-instance arrays the timed path's caller received in the last timed step, one
+    <out_dir>/<name>.npy each in float64. Beyond DUMP_BYTES the same seeded sample of instances is taken from
+    every array; instance.npy lists the instances written."""
+    batch = len(arrays["cost"])
+    per_instance = 8 * (1 + sum(a[0].size for a in arrays.values()))
+    keep = min(batch, (DUMP_BYTES - 4096) // per_instance)  # 4096: room for the .npy headers
+    idx = np.arange(batch) if keep == batch else np.sort(np.random.default_rng(0).choice(batch, keep, replace=False))
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in dict({k: v[idx] for k, v in arrays.items()}, instance=idx).items():
+        np.save(os.path.join(out_dir, name + ".npy"), a.astype(np.float64))
+
+
 def sv_uses_tmem(n, batch):
     """The library's storage policy (DESIGN.md §4): tensor memory for n_max >= 64."""
     return n >= 64
 
 
 def measure_cold(args, hb, option_bits, steps, warmup, e2e_steps, local_rank, world, dev, gather=True, clocks=False,
-                 inflight=1):
+                 inflight=1, dump_dir=None):
     """Cold solves of this rank's batch `hb`: device-resident value, end-to-end value, kernel time.
     inflight = 2: consecutive steps alternate between two handles on two streams, so the next batch's CTAs take
     over SMs as the previous batch's persistent CTAs run out of work (iteration counts are heavy-tailed: 10 % of a
-    lone launch is tail). Every step is still one full batch; the timed region covers all of them."""
+    lone launch is tail). Every step is still one full batch; the timed region covers all of them.
+    dump_dir: rank 0 writes the last timed step's results there (dump_outputs)."""
     import torch
     from path_optimizer_2_b200 import solver
     params = abi.default_params(reserved=option_bits)
@@ -565,6 +585,9 @@ def measure_cold(args, hb, option_bits, steps, warmup, e2e_steps, local_rank, wo
     total_ms = reduce_max(my_ms, dev, world)
     last = (steps - 1) % K
     status, iters = outs[last][2].cpu().numpy(), outs[last][3].cpu().numpy()
+    if dump_dir and int(os.environ.get("RANK", "0")) == 0:
+        dump_outputs(dump_dir, {"sol": outs[last][0].cpu().numpy(), "cost": outs[last][1].cpu().numpy(),
+                                "status": status, "iters": iters})
     for k in range(K):  # every handle solved the same batch: identical results
         assert np.array_equal(outs[k][2].cpu().numpy(), status) or steps <= k
     if pipes[last]:  # the gathered table holds every rank's records; this rank's block must equal its own results
@@ -631,11 +654,12 @@ def measure_cold(args, hb, option_bits, steps, warmup, e2e_steps, local_rank, wo
             "info": info, "params": params, "flushed": flush is not None, "steps": steps}
 
 
-def run_receding(args, rank, local_rank, world, dev):
+def run_receding(args, rank, local_rank, world, dev, dump_dir=None):
     """BASELINE configs[4]: receding-horizon warm re-solves (SURVEY.md §8d config 5). One step =
     one tick: advance the window by one knot (pqp_advance_window_device, one launch),
     re-linearise about the previous solution, warm re-solve with max_iter = 50 through
-    pqp_resolve_device; x, z, y, rho stay resident in the handle between ticks."""
+    pqp_resolve_device; x, z, y, rho stay resident in the handle between ticks.
+    dump_dir: rank 0 writes the last timed tick's results there (dump_outputs)."""
     import torch
     from path_optimizer_2_b200 import solver
 
@@ -702,6 +726,8 @@ def run_receding(args, rank, local_rank, world, dev):
     value = world * B * args.steps / (total_ms * 1e-3)
     status = d_status.cpu().numpy()
     iters = d_iters.cpu().numpy()
+    if dump_dir and rank == 0:
+        dump_outputs(dump_dir, {"sol": d_sol.cpu().numpy(), "cost": d_cost.cpu().numpy(), "status": status, "iters": iters})
     kms = gather_scalars(kernel_ms, dev, world)
 
     # e2e: the same tick through the host-pointer call (pinned host buffers, H2D + D2H timed);
@@ -772,10 +798,10 @@ def dropin_single_path(n=120, plans=200):
     hb = lines.to_host_batch(bnd[None], np.array([nv], dtype=np.int32))
     nn = int(hb.n[0])
     ref = np.stack([lines.states[0][1], lines.states[0][2], lines.states[0][3]])
-    path = os.path.join(ROOT, "gpurun_out", "bench_dropin_instance.txt")
-    os.makedirs(os.path.dirname(path), exist_ok=True)
-    test_dropin._write_instance(path, hb.knots[0], hb.inst[0], nn, ref, 0.0, constraint_end_heading=0)
-    out = subprocess.run([exe, path, str(plans)], capture_output=True, text=True, check=True).stdout.strip().split("\n")
+    with tempfile.TemporaryDirectory() as tmp:  # the tree may be read-only
+        path = os.path.join(tmp, "dropin_instance.txt")
+        test_dropin._write_instance(path, hb.knots[0], hb.inst[0], nn, ref, 0.0, constraint_end_heading=0)
+        out = subprocess.run([exe, path, str(plans)], capture_output=True, text=True, check=True).stdout.strip().split("\n")
     tok = out[0].split()
     if tok[0] != "plans":
         return {"error": out[0]}
@@ -933,7 +959,13 @@ def main():
                     help="cold: BASELINE configs[2]/[3] (default); receding: configs[4], warm re-solves with a "
                          "50-iteration cap on a window that advances one knot per step; sharedmap: configs[1], "
                          "1024 paths x 120 knots through the shared obstacle map")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last timed step returned for rank 0's batch (solution, "
+                         "cost, status, iterations) as DIR/<name>.npy in float64, at most 64 MB in all (a seeded "
+                         "sample of instances beyond that; DIR/instance.npy lists them)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.workload == "receding" and args.batch == 8192:
         args.batch = 512  # configs[4]: 4096 instances over 8 GPUs
     if args.workload == "sharedmap":
@@ -963,7 +995,7 @@ def main():
         dist.init_process_group("nccl", device_id=dev)
 
     if args.workload == "receding":
-        line = run_receding(args, rank, local_rank, world, dev)
+        line = run_receding(args, rank, local_rank, world, dev, dump_dir=args.dump_outputs)
         if rank == 0:
             print(json.dumps(line))
         if world > 1:
@@ -976,7 +1008,7 @@ def main():
     extras.pop("_lines", None)
     extras.pop("_dmap", None)
     r = measure_cold(args, hb, args.option_bits, args.steps, args.warmup, args.e2e_steps or args.steps, local_rank,
-                     world, dev, gather=True, clocks=True, inflight=args.inflight)
+                     world, dev, gather=True, clocks=True, inflight=args.inflight, dump_dir=args.dump_outputs)
     fp64, sec = (None, None) if args.no_secondary else secondary(args, rank, local_rank, world, dev, hb)
 
     if rank == 0:

@@ -10,10 +10,11 @@
 
 // Two builds of this file (tests/test_dropin.py):
 //   dropin_test       against tests/cpp/ref_stub.hpp (stand-ins; builds anywhere);
-//   dropin_test_real  with -DPQP_TEST_REAL_TYPES -I/root/reference/include, i.e. against the reference's
+//   dropin_test_real  with -DPQP_TEST_REAL_TYPES -I oracle/_ref/include, i.e. against the reference's
 //                     OWN State / SlState / VehicleStateBound (include/data_struct/data_struct.hpp) and
-//                     VehicleState (vehicle_state_frenet.hpp, its .cpp compiled from where it lies). Only
-//                     the reference's ReferencePath cannot be compiled here (it needs grid_map / glog), so
+//                     VehicleState (vehicle_state_frenet.hpp and an object of its .cpp), as staged from
+//                     a checkout of the original project by `make -C oracle ref`. Only
+//                     the reference's ReferencePath cannot be compiled standalone (it needs grid_map / glog), so
 //                     a holder with the three accessors the solver reads carries the real element types.
 #include "../../include/pqp_base_solver.hpp"
 #ifdef PQP_TEST_REAL_TYPES

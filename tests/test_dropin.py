@@ -18,23 +18,27 @@ BIN = os.path.join(ROOT, "tests", "cpp", "dropin_test")
 
 
 BIN_REAL = BIN + "_real"
-REF = "/root/reference"
+REF_STAGED = os.path.join(ROOT, "oracle", "_ref")
 
 
 def _build(real=False):
-    """real=True: bind the drop-in to the reference's OWN boundary types (data_struct.hpp,
-    vehicle_state_frenet.{hpp,cpp} compile standalone, SURVEY.md §8c). Only possible where
-    /root/reference exists (the CPU box); the binary is git-ignored but travels to the GPU box."""
+    """real=True: bind the drop-in to the original project's OWN boundary types (data_struct.hpp,
+    vehicle_state_frenet.{hpp,cpp} compile standalone, SURVEY.md §8c), staged in oracle/_ref/ by
+    `make -C oracle ref` (build() does that where a checkout of that project is readable); None where
+    nothing was staged."""
     solver.build_library()
     out = BIN_REAL if real else BIN
     src = os.path.join(ROOT, "tests", "cpp", "dropin_test.cpp")
     deps = [src, os.path.join(ROOT, "include", "pqp_base_solver.hpp"), os.path.join(ROOT, "tests", "cpp", "ref_stub.hpp"),
             solver.LIB_PATH]
-    if real and not os.path.isdir(REF):
-        return out if os.path.exists(out) else None
+    if real:
+        staged = [os.path.join(REF_STAGED, "include", "data_struct", h) for h in ("data_struct.hpp", "vehicle_state_frenet.hpp")]
+        staged.append(os.path.join(REF_STAGED, "vehicle_state_frenet.o"))
+        if not all(os.path.exists(f) for f in staged):
+            return None
+        deps += staged
     if not os.path.exists(out) or any(os.path.getmtime(d) > os.path.getmtime(out) for d in deps):
-        extra = ["-DPQP_TEST_REAL_TYPES", "-I", os.path.join(REF, "include"), "-w",
-                 os.path.join(REF, "src", "data_struct", "vehicle_state_frenet.cpp")] if real else ["-Wall"]
+        extra = ["-DPQP_TEST_REAL_TYPES", "-I", os.path.join(REF_STAGED, "include"), "-w", staged[-1]] if real else ["-Wall"]
         subprocess.check_call(["g++", "-std=c++11", "-O1", "-o", out, src] + extra + [
             solver.LIB_PATH, "-Wl,-rpath," + os.path.dirname(solver.LIB_PATH)])
     return out
@@ -55,7 +59,7 @@ def _write_instance(path, knots, inst, n, ref, target_heading, constraint_end_he
 def test_dropin_compiles_and_fails_loudly_without_gpu(tmp_path, real):
     exe = _build(real)
     if exe is None:
-        pytest.skip("the reference tree is not present on this box")
+        pytest.skip("the drop-in against the original project's types was not built (nothing staged in oracle/_ref)")
     try:
         import torch
         if torch.cuda.is_available():
@@ -75,7 +79,7 @@ def test_dropin_matches_python_binding(tmp_path, real):
     from oracle import oracle
     exe = _build(real)
     if exe is None:
-        pytest.skip("dropin_test_real was not built on the CPU box")
+        pytest.skip("the drop-in against the original project's types was not built (nothing staged in oracle/_ref)")
     params = abi.default_params()
     for idx in range(3):
         knots, inst, n, ref = synthetic.make_instance(3, idx, 120)
